@@ -2,7 +2,7 @@
 """Benchmark of the DD3D inference hot path (contract: see the task statement / DESIGN.md "Measurement").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload v2_99|dla34|nusc_v2_99]
-                    [--batch B] [--dtype bf16|fp16] [--input mapped|raw] [--sweep 8,16,32,64]
+                    [--batch B] [--dtype bf16|fp16] [--input mapped|raw] [--sweep 8,16,32,64] [--dump-outputs DIR]
 
 A step = one DD3D.forward over one batch of synthetic images per GPU:
   v2_99 (default, the config BASELINE.json's metric is quoted on): V2-99 DD3D, 32 x 900x1600 per GPU;
@@ -17,6 +17,8 @@ forward of step k+1 and no host synchronisation happens inside the timed region.
 it needs detectron2/pytorch3d, not installable offline) on rank 0 with all host threads, following BASELINE.md 3
 (batch = min(B, 8) images per forward, bounded so that the run ends within minutes).
 `--sweep` (BASELINE.json configs[4]): per-GPU batch sweep; prints one JSON line per batch size.
+`--dump-outputs DIR` (rank 0): the detections of the last timed step of every workload the run times, one float .npy per
+Instances field (see dump_detections), so that two builds can be compared output for output on identical seeded inputs.
 """
 import argparse
 import ctypes as C
@@ -131,6 +133,37 @@ def pick_threads():
     return best
 
 
+DUMP_BUDGET = {"bytes": 64 << 20}  # all arrays of one --dump-outputs run together
+
+
+def dump_detections(dirname, prefix, out, counts, glob=None):
+    """Writes one step's packed [B][cap] dd3d_det buffer as the Instances fields a caller receives (DD3DB200._wrap), each
+    padded to [B, cap, ...] with zeros past counts[b], float32 (float64 for the integer fields and counts).  If the arrays
+    of all B images do not fit what is left of DUMP_BUDGET, only those of the first images that fit are written."""
+    import numpy as np
+    import torch
+    out, counts = out.cpu(), counts.cpu()
+    B, cap = out.shape[:2]
+    words = out.clone()
+    words[torch.arange(cap)[None, :] >= counts[:, None].long()] = 0
+    f, i = words, words.view(torch.int32)
+    fields = {"pred_boxes": f[..., 0:4], "scores": f[..., 4], "scores_3d": f[..., 5], "pred_classes": i[..., 6].double(),
+              "fpn_levels": i[..., 7].double(), "quat": f[..., 8:12], "proj_ctr": f[..., 12:14], "depth": f[..., 14],
+              "size": f[..., 15:18], "locations": f[..., 18:20]}
+    if glob is not None:  # NuscenesDD3D
+        g = glob.cpu().clone()
+        g[torch.arange(cap)[None, :] >= counts[:, None].long()] = 0
+        fields.update(pred_attributes=i[..., 21].double(), pred_speeds=f[..., 22], pred_boxes3d_global=g)
+    per_image = sum(v[0].numel() * v.element_size() for v in fields.values()) + 8
+    n = min(B, DUMP_BUDGET["bytes"] // per_image)
+    assert n > 0, "--dump-outputs: 64 MB budget exhausted"
+    DUMP_BUDGET["bytes"] -= n * per_image
+    fields["counts"] = counts.double()
+    os.makedirs(dirname, exist_ok=True)
+    for name, v in fields.items():
+        np.save(os.path.join(dirname, f"{prefix}{name}.npy"), v[:n].contiguous().numpy())
+
+
 def cpu_model():
     try:
         with open("/proc/cpuinfo") as f:
@@ -191,7 +224,8 @@ def run_reference(args, rank):
     print(json.dumps(line), flush=True)
 
 
-def run_workload(args, workload, batch, rank, local_rank, world, gatherer_cache, with_cpu=True, steps=None, warmup=None):
+def run_workload(args, workload, batch, rank, local_rank, world, gatherer_cache, with_cpu=True, steps=None, warmup=None,
+                 dump_prefix=""):
     """Times one workload on this rank's GPU; returns the JSON line (dict).  All ranks must call it together."""
     import torch
     import torch.distributed as dist
@@ -399,6 +433,9 @@ def run_workload(args, workload, batch, rank, local_rank, world, gatherer_cache,
         return finish_timing(e0, e1, tag), clocks
 
     ms_dev, clocks = timed(step_device, "value", ClockSampler(local_rank))
+    if args.dump_outputs and rank == 0:  # before the e2e legs below reuse the buffers
+        last = (state["k"] - 1) & 1
+        dump_detections(args.dump_outputs, dump_prefix, packed[last].out, packed[last].counts, d_glob if nusc else None)
     ms_host, _ = timed(step_host, "e2e_serial")
     ms_host_serial = ms_host
     if not nusc and not raw_mode:  # double-buffered host path (H2D of the next step overlaps this step's kernels)
@@ -519,6 +556,9 @@ def main():
     ap.add_argument("--input", default="mapped", choices=["mapped", "raw"],
                     help="raw: steps start from raw HWC uint8 dataset images (dd3d_forward_raw: ResizeShortestEdge to "
                          "INPUT.RESIZE.MIN_SIZE_TEST + intrinsics rescale on the GPU); not the BASELINE configuration")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the detections of the last timed step as DIR/<field>.npy (the DLA-34 leg of the default "
+                         "run: secondary_<field>; --sweep: batch<B>_<field>)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -538,17 +578,18 @@ def main():
     gatherers = {}
     if args.sweep:
         for b in [int(v) for v in args.sweep.split(",")]:
-            line = run_workload(args, args.workload, b, rank, local_rank, world, gatherers, with_cpu=False)
+            line = run_workload(args, args.workload, b, rank, local_rank, world, gatherers, with_cpu=False,
+                                dump_prefix=f"batch{b}_")
             if rank == 0:
                 print(json.dumps(line), flush=True)
     else:
         line = run_workload(args, args.workload, args.batch, rank, local_rank, world, gatherers)
         default_run = (args.workload == "v2_99" and not args.batch and args.dtype == "bf16" and args.input == "mapped")
         if default_run and world == 1 and not args.no_secondary:
-            # BASELINE.json configs[1] (DLA-34 bf16, batch 8, 384x1280) measured in the same process, so that the driver's
-            # single `bench.py` run records it too
-            sec = run_workload(args, "dla34", 0, rank, local_rank, world, gatherers, with_cpu=False, steps=max(args.steps, 20),
-                               warmup=max(args.warmup, 5))
+            # BASELINE.json configs[1] (DLA-34 bf16, batch 8, 384x1280) measured in the same process, so that a single
+            # `bench.py` run records it too
+            sec = run_workload(args, "dla34", 0, rank, local_rank, world, gatherers, with_cpu=False,
+                               warmup=max(args.warmup, 5), dump_prefix="secondary_")
             line["secondary"] = {k: sec[k] for k in ("metric", "value", "unit", "ms_per_step", "steps", "dtype", "config",
                                                       "clocks", "e2e", "gpu_launches", "roofline", "kernels_ms_per_step")}
         if rank == 0:

@@ -9,6 +9,7 @@ dd3d_b200.synthetic.make_inputs):
   golden_<arch>.npz : per image b -> boxes, scores, scores_3d, classes, levels, locations, quat, proj_ctr, depth, size,
                       tvec (post NMS / top-k / postprocess), plus the case description.
   kat_boxes3d.npz   : known-answer vector for predictions_to_boxes3d (fcos3d.py:16-52) from SURVEY.md 8c.
+  reference_checks.npz, reference_configs.json : see gen_reference_checks (`--checks` writes only these two).
 """
 import os
 import sys
@@ -185,11 +186,118 @@ def gen_dd3d_goldens(names, out_dir):
         np.savez_compressed(os.path.join(out_dir, f"golden_{arch}.npz"), **blob)
 
 
+def instances_blob(prefix, inst):
+    """The fields of one reference Instances as arrays "<prefix>/<field>" (3-D fields only when the model predicts them)."""
+    blob = {f"{prefix}/boxes": inst.pred_boxes.tensor.numpy(), f"{prefix}/scores": inst.scores.numpy(),
+            f"{prefix}/classes": inst.pred_classes.numpy(), f"{prefix}/levels": inst.fpn_levels.numpy(),
+            f"{prefix}/locations": inst.locations.numpy(), f"{prefix}/has_box3d": np.array(inst.has("pred_boxes3d"))}
+    if inst.has("pred_boxes3d"):
+        b3 = inst.pred_boxes3d
+        blob.update({f"{prefix}/scores_3d": inst.scores_3d.numpy(), f"{prefix}/quat": b3.quat.numpy(),
+                     f"{prefix}/depth": b3.depth.numpy().reshape(-1), f"{prefix}/size": b3.size.numpy(),
+                     f"{prefix}/tvec": b3.tvec.numpy()})
+    return blob
+
+
+def inventory_blob(prefix, model):
+    """The reference model's state_dict inventory: sorted keys and their shapes ("64x3x7x7")."""
+    sd = model.state_dict()
+    keys = sorted(sd)
+    return {f"{prefix}/keys": np.array(keys), f"{prefix}/shapes": np.array(["x".join(map(str, sd[k].shape)) for k in keys])}
+
+
+def gen_reference_checks(out_dir):
+    """reference_checks.npz / reference_configs.json: what the oracle and config checks of the CPU suite compare against,
+    recorded from the reference itself -- its parameter inventory and forward under the decode / head switches
+    (tests/test_cpu_oracle.py), its BEV NMS / sample aggregation / intrinsics rescale on the seeded cases of
+    tests/test_bev_nms.py, test_nuscenes.py, test_input_pipeline.py, its model attributes and KITTI3DEvaluator.process()
+    rows for the dla34 golden case (tests/boundary_probe.py), and its four DD3D experiments composed by
+    tests/hydra_lite.py (tests/test_config_vs_reference.py)."""
+    import json
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from hydra_lite import compose_experiment
+    from test_bev_nms import _random_case
+    from test_config_vs_reference import EXPERIMENTS
+    from test_cpu_oracle import FLAG_CASES, HEAD_CASES, apply_flags, apply_head_flags
+    from test_nuscenes import aggregate_case
+
+    configs = {e: compose_experiment(os.path.join(ref_standin.REFERENCE_ROOT, "configs"), e) for e, _ in EXPERIMENTS}
+    with open(os.path.join(out_dir, "reference_configs.json"), "w") as f:
+        json.dump(configs, f, indent=1, sort_keys=True)
+        f.write("\n")
+
+    blob = {}
+    small = make_inputs(1, 128, 256, 721.5, seed_base=7)
+    runs = [(f"inventory_{arch}", get_cfg(arch, CASES[arch][0])) for arch in CASES]
+    for i, flags in enumerate(FLAG_CASES):
+        runs.append((f"flags{i}", apply_flags(get_cfg("dla34", "kitti_3d"), flags)))
+    for i, flags in enumerate(HEAD_CASES):
+        runs.append((f"head{i}", apply_head_flags(get_cfg("dla34", "kitti_3d"), flags)))
+    for name, cfg in runs:
+        if not name.startswith("inventory"):
+            cfg.DD3D.FCOS2D.INFERENCE.PRE_NMS_THRESH = 0.03
+        model = ref_standin.build_reference_model(cfg).eval()
+        blob.update(inventory_blob(name, model))
+        model.load_state_dict(make_state_dict(cfg))
+        with torch.no_grad():
+            inst = model(small)[0]["instances"]
+        blob.update(instances_blob(name, inst))
+        print(name, "detections", len(inst))
+
+    for c in range(4):
+        det, pq, pt = _random_case(7 + c, 40 + 5 * c)
+        blob[f"bev{c}/keep"] = reference_bev_keep(det, pq, pt, 0.3)[0].numpy()
+    dets, gids, poses = aggregate_case(3)
+    for i, (keep, _, _) in enumerate(reference_sample_aggregate(dets, gids, poses, 0.3, 200)):
+        blob[f"aggregate/keep{i}"] = keep.numpy()
+    from tridet.data.augmentations.resize_transform import ResizeTransform
+    K = np.float32([[1266.4, 0, 816.3], [0, 1266.4, 491.5], [0, 0, 1]])
+    for i, ((h, w), (nh, nw)) in enumerate([((900, 1600), (896, 1593)), ((375, 1242), (384, 1272))]):
+        blob[f"intrinsics{i}/K"] = ResizeTransform(h, w, nh, nw).apply_intrinsics(K)
+
+    # boundary: the reference DD3D's attributes and its evaluator's rows for its own detections on the dla34 golden case
+    ref_standin.install_evaluator_stubs()
+    from detectron2.data.catalog import DatasetCatalog, MetadataCatalog
+    from types import SimpleNamespace
+    from tridet.evaluators.kitti_3d_evaluator import KITTI3DEvaluator
+    cfg = get_cfg("dla34", "kitti_3d")
+    model = ref_standin.build_reference_model(cfg).eval()
+    model.load_state_dict(make_state_dict(cfg))
+    for attr in ("postprocess_in_inference", "do_nms", "do_bev_nms", "bev_nms_iou_thresh", "only_box2d", "num_classes"):
+        blob[f"boundary/{attr}"] = np.array(getattr(model, attr))
+    blob["boundary/size_divisibility"] = np.array(model.backbone.size_divisibility)
+    inputs = case_inputs("dla34")
+    for i, x in enumerate(inputs):
+        x["file_name"], x["image_id"] = f"img{i:06d}.png", i
+    names = ["Car", "Pedestrian", "Cyclist", "Van", "Truck"]
+    DatasetCatalog.register("kitti_probe", lambda: [{"file_name": x["file_name"]} for x in inputs])
+    MetadataCatalog.register("kitti_probe", SimpleNamespace(thing_classes=names, contiguous_id_to_name=dict(enumerate(names))))
+    with torch.no_grad():
+        outs = model(inputs)
+    for b, o in enumerate(outs):
+        blob[f"boundary/image_size{b}"] = np.array(o["instances"].image_size)
+        blob[f"boundary/fields{b}"] = np.array(sorted(o["instances"].get_fields()))
+    ev = KITTI3DEvaluator("kitti_probe", iou_thresholds=[0.5, 0.7])
+    ev.reset()
+    ev.process(inputs, outs)
+    rows = ev._predictions_as_json
+    blob["boundary/category"] = np.array([r["category"] for r in rows])
+    blob["boundary/file_name"] = np.array([r["file_name"] for r in rows])
+    blob["boundary/image_id"] = np.array([r["image_id"] for r in rows])
+    for k in ("category_id", "bbox3d", "bbox", "score", "score_3d"):
+        blob[f"boundary/{k}"] = np.array([r[k] for r in rows])
+    print("boundary: evaluator rows", len(rows))
+    np.savez_compressed(os.path.join(out_dir, "reference_checks.npz"), **blob)
+
+
 def main():
     out_dir = os.path.join(ROOT, "tests", "golden")
     os.makedirs(out_dir, exist_ok=True)
     if "--full" in sys.argv:  # only the BASELINE-shape cases (a V2-99 900x1600 reference forward takes ~10 s here)
         gen_dd3d_goldens(list(FULL_CASES), out_dir)
+        return
+    if "--checks" in sys.argv:  # only reference_checks.npz / reference_configs.json
+        gen_reference_checks(out_dir)
         return
     gen_dd3d_goldens(list(CASES) + list(FULL_CASES), out_dir)
 
@@ -291,6 +399,7 @@ def main():
              depth_in=depth.numpy(), size_in=size.numpy(), loc=loc.numpy(), canon=canon.numpy(), quat=b3.quat.numpy(),
              proj_ctr=b3.proj_ctr.numpy(), depth=b3.depth.numpy(), size=b3.size.numpy(), tvec=b3.tvec.numpy())
     print("KAT quat", b3.quat.numpy(), "tvec", b3.tvec.numpy())
+    gen_reference_checks(out_dir)
 
 
 if __name__ == "__main__":

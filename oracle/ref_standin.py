@@ -681,6 +681,7 @@ def _mod(name, **attrs):
 
 
 _INSTALLED = False
+_THIRD_PARTY_INSTALLED = False
 
 
 # ----------------------------------------------------------------------------------------------
@@ -864,16 +865,16 @@ def apply_augmentations(augmentations, image):
     return image, TransformList(tfms)
 
 
-def install(reference_root=REFERENCE_ROOT):
-    """Put the stand-in modules and the reference's `tridet` package on the import path."""
-    global _INSTALLED
-    if _INSTALLED:
+def _noop(*a, **k):
+    return None
+
+
+def install_third_party():
+    """Put the stand-in detectron2 / fvcore / pytorch3d / pyquaternion / mpi4py modules on the import path."""
+    global _THIRD_PARTY_INSTALLED
+    if _THIRD_PARTY_INSTALLED:
         return
-    _INSTALLED = True
-
-    def _noop(*a, **k):
-        return None
-
+    _THIRD_PARTY_INSTALLED = True
     _mod("detectron2")
     _mod("detectron2.config", configurable=configurable)
     _mod("detectron2.layers", Conv2d=Conv2d, get_norm=get_norm, cat=cat, batched_nms=batched_nms,
@@ -906,6 +907,15 @@ def install(reference_root=REFERENCE_ROOT):
 
     _mod("pyquaternion", Quaternion=Quaternion)
     _mod("mpi4py", MPI=types.SimpleNamespace(COMM_WORLD=None))
+
+
+def install(reference_root=REFERENCE_ROOT):
+    """Put the stand-in modules and the reference's `tridet` package on the import path."""
+    global _INSTALLED
+    if _INSTALLED:
+        return
+    _INSTALLED = True
+    install_third_party()
 
     # The reference's package __init__ files pull in the nuScenes devkit / TTA wrappers; stub the
     # package nodes (not the hot-path modules) so `tridet.modeling.dd3d.core` imports verbatim.

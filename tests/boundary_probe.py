@@ -1,19 +1,20 @@
-"""Run as a subprocess by tests/test_boundary_reference_plumbing.py (build container only: needs /root/reference).
+"""Run as a subprocess by tests/test_boundary_reference_plumbing.py.
 
-Drives the B200 mirror through the REFERENCE's own plumbing, everything imported unmodified from /root/reference under
-the third-party stand-in (oracle/ref_standin.py):
-
+Drives the B200 mirror through the plumbing the reference's scripts use, with the detectron2 stand-in of
+oracle/ref_standin.py installed in place of detectron2, and checks it against what the reference produced on the dla34
+golden case (tests/golden/reference_checks.npz "boundary/*", recorded by oracle/gen_golden.py):
  1. registry: with the stand-in installed BEFORE dd3d_b200 is imported, `dd3d_b200.meta_arch` registers DD3DB200 /
-    NuscenesDD3DB200 in the same META_ARCH_REGISTRY the reference's DD3D registers in (core.py:18), and the model is built
-    the way scripts/train.py:48 -> detectron2 build_model does: META_ARCH_REGISTRY.get(cfg.MODEL.META_ARCHITECTURE)(cfg),
-    .to(cfg.MODEL.DEVICE) -- selected purely by the config string;
- 2. types: the Instances it returns are the (stand-in) detectron2 Instances / Boxes and the reference's own Boxes3D;
- 3. evaluator: the reference's KITTI3DEvaluator.process() (kitti_3d_evaluator.py:66-123: per-detection iteration of
-    pred_boxes3d, .vectorize(), convert_3d_box_to_kitti) consumes those outputs; its JSON / KITTI rows are identical to the
-    ones it produces from the reference model's own outputs for the same detections.
+    NuscenesDD3DB200 in detectron2's META_ARCH_REGISTRY (where the reference's DD3D registers, core.py:18), and the model
+    is built the way scripts/train.py:48 -> detectron2 build_model does: META_ARCH_REGISTRY.get(cfg.MODEL.META_ARCHITECTURE)
+    (cfg), .to(cfg.MODEL.DEVICE) -- selected purely by the config string; the attributes do_test / DD3DWithTTA poke equal
+    the reference DD3D's;
+ 2. types: the Instances it returns are detectron2's Instances / Boxes, with the reference's fields and image sizes;
+ 3. evaluator: what the reference's KITTI3DEvaluator.process() (kitti_3d_evaluator.py:66-123) reads from them per
+    detection -- class, pred_boxes3d[i].vectorize(), the XYWH 2-D box, scores, scores_3d -- equals the rows it wrote from
+    the reference model's own outputs (its KITTI rows are a function of the same values).
 The detections fed through DD3DB200._wrap (the product code that turns the C ABI's packed [B][cap][24] buffer into
-Instances) are the reference DD3D's own detections on the dla34 golden case, packed into the C-ABI layout -- there is no GPU
-in the build container, and no reference on the GPU box.
+Instances) are the reference DD3D's own detections on the dla34 golden case (tests/golden/golden_dla34.npz), packed into
+the C-ABI layout -- the wrapping needs no GPU.
 """
 import os
 import sys
@@ -25,14 +26,15 @@ ROOT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..")
 sys.path.insert(0, os.path.abspath(ROOT))
 from oracle import ref_standin  # noqa: E402
 
-ref_standin.install_evaluator_stubs()
+ref_standin.install_third_party()
 from detectron2.modeling.meta_arch.build import META_ARCH_REGISTRY  # noqa: E402  (stand-in registry)
-from tridet.modeling.dd3d.core import DD3D as RefDD3D  # noqa: E402  (registers the reference's DD3D)
 import dd3d_b200.meta_arch as ma  # noqa: E402  registers DD3DB200 / NuscenesDD3DB200
 from dd3d_b200 import lib  # noqa: E402
 from dd3d_b200.config import get_cfg  # noqa: E402
 from dd3d_b200.synthetic import make_state_dict  # noqa: E402
 from oracle.gen_golden import case_inputs  # noqa: E402
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def build_model(cfg):
@@ -42,52 +44,46 @@ def build_model(cfg):
     return model
 
 
-def pack_words(outputs, cap):
-    """reference Instances -> the C ABI's [B][cap][24] fp32 words + counts (include/dd3d_b200.h dd3d_det)."""
-    B = len(outputs)
-    out = torch.zeros(B, cap, lib.DET_WORDS, dtype=torch.float32)
+def pack_words(golden, nimg, cap):
+    """golden_dla34.npz detections -> the C ABI's [B][cap][24] fp32 words + counts (include/dd3d_b200.h dd3d_det)."""
+    out = torch.zeros(nimg, cap, lib.DET_WORDS, dtype=torch.float32)
     oi = out.view(torch.int32)
-    counts = torch.zeros(B, dtype=torch.int32)
-    for b, o in enumerate(outputs):
-        inst = o["instances"]
-        n = len(inst)
+    counts = torch.zeros(nimg, dtype=torch.int32)
+    for b in range(nimg):
+        n = golden[f"boxes{b}"].shape[0]
         counts[b] = n
-        b3 = inst.pred_boxes3d
-        out[b, :n, 0:4] = inst.pred_boxes.tensor
-        out[b, :n, 4] = inst.scores
-        out[b, :n, 5] = inst.scores_3d
-        oi[b, :n, 6] = inst.pred_classes.to(torch.int32)
-        oi[b, :n, 7] = inst.fpn_levels.to(torch.int32)
-        out[b, :n, 8:12] = b3.quat
-        out[b, :n, 12:14] = b3.proj_ctr
-        out[b, :n, 14] = b3.depth.reshape(-1)
-        out[b, :n, 15:18] = b3.size
-        out[b, :n, 18:20] = inst.locations
+        out[b, :n, 0:4] = torch.from_numpy(golden[f"boxes{b}"])
+        out[b, :n, 4] = torch.from_numpy(golden[f"scores{b}"])
+        out[b, :n, 5] = torch.from_numpy(golden[f"scores_3d{b}"])
+        oi[b, :n, 6] = torch.from_numpy(golden[f"classes{b}"]).to(torch.int32)
+        oi[b, :n, 7] = torch.from_numpy(golden[f"levels{b}"]).to(torch.int32)
+        out[b, :n, 8:12] = torch.from_numpy(golden[f"quat{b}"])
+        out[b, :n, 12:14] = torch.from_numpy(golden[f"proj_ctr{b}"])
+        out[b, :n, 14] = torch.from_numpy(golden[f"depth{b}"]).reshape(-1)
+        out[b, :n, 15:18] = torch.from_numpy(golden[f"size{b}"])
+        out[b, :n, 18:20] = torch.from_numpy(golden[f"locations{b}"])
     return out, counts
 
 
 def main():
+    ref = np.load(os.path.join(GOLDEN, "reference_checks.npz"))
+    ref = {k.split("/", 1)[1]: v for k, v in ref.items() if k.startswith("boundary/")}
+
     # ---- 1. registry / build_model by config string
-    assert META_ARCH_REGISTRY.get("DD3D") is RefDD3D
     assert META_ARCH_REGISTRY.get("DD3DB200") is ma.DD3DB200
     assert META_ARCH_REGISTRY.get("NuscenesDD3DB200") is ma.NuscenesDD3DB200
     cfg = get_cfg("dla34", "kitti_3d")
+    assert cfg.MODEL.META_ARCHITECTURE == "DD3D"  # the experiment's own string selects the reference's DD3D
     cfg.MODEL.DEVICE = "cpu"
-    sd = make_state_dict(cfg)
-    ref_model = build_model(cfg).eval()  # MODEL.META_ARCHITECTURE == "DD3D": the reference's own class
-    assert type(ref_model) is RefDD3D
-    ref_model.load_state_dict(sd)
-    cfg_b = get_cfg("dla34", "kitti_3d")
-    cfg_b.MODEL.DEVICE = "cpu"
-    cfg_b.MODEL.META_ARCHITECTURE = "DD3DB200"
-    model = build_model(cfg_b)
+    cfg.MODEL.META_ARCHITECTURE = "DD3DB200"
+    model = build_model(cfg)
     assert type(model) is ma.DD3DB200
     for attr in ("postprocess_in_inference", "do_nms", "do_bev_nms", "bev_nms_iou_thresh", "only_box2d", "num_classes",
                  "device"):  # what do_test / DD3DWithTTA poke (scripts/train.py:206-209, test_time_augmentation.py:107)
         assert hasattr(model, attr), attr
-        assert getattr(model, attr) == getattr(ref_model, attr) or attr == "device", attr
-    assert model.backbone.size_divisibility == ref_model.backbone.size_divisibility
-    res = model.load_state_dict(ref_model.state_dict())  # Checkpointer(model).load(): the reference's own key set
+        assert attr == "device" or getattr(model, attr) == ref[attr].item(), attr
+    assert model.backbone.size_divisibility == ref["size_divisibility"].item()
+    res = model.load_state_dict(make_state_dict(cfg))  # the reference's key set (tests/test_cpu_oracle.py inventory)
     assert not res.missing_keys and not res.unexpected_keys
     try:
         model([{"image": torch.zeros(3, 8, 8, dtype=torch.uint8), "intrinsics": torch.eye(3) * 2}])
@@ -95,51 +91,38 @@ def main():
     except RuntimeError as e:
         assert "no CPU path" in str(e)
 
-    # ---- 2. + 3. reference evaluator on the mirror's output containers
-    from detectron2.data.catalog import DatasetCatalog, MetadataCatalog
-    from types import SimpleNamespace
+    # ---- 2. + 3. the mirror's output containers vs what the reference evaluator read from the reference's own
     inputs = case_inputs("dla34")
-    for i, x in enumerate(inputs):
-        x["file_name"], x["image_id"] = f"img{i:06d}.png", i
-    names = ["Car", "Pedestrian", "Cyclist", "Van", "Truck"]
-    DatasetCatalog.register("kitti_probe", lambda: [{"file_name": x["file_name"]} for x in inputs])  # test split: no GT
-    MetadataCatalog.register("kitti_probe", SimpleNamespace(thing_classes=names,
-                                                            contiguous_id_to_name=dict(enumerate(names))))
-    from tridet.evaluators.kitti_3d_evaluator import KITTI3DEvaluator
-    with torch.no_grad():
-        ref_out = ref_model(inputs)
-    assert sum(len(o["instances"]) for o in ref_out) > 10
-    words, counts = pack_words(ref_out, model._desc.out_cap)
+    golden = np.load(os.path.join(GOLDEN, "golden_dla34.npz"))
+    words, counts = pack_words(golden, len(inputs), model._desc.out_cap)
+    assert int(counts.sum()) > 10
     K = torch.stack([x["intrinsics"] for x in inputs]).reshape(len(inputs), 9)
     sizes = torch.tensor([[x["image"].shape[-2], x["image"].shape[-1], x.get("height", x["image"].shape[-2]),
                            x.get("width", x["image"].shape[-1])] for x in inputs], dtype=torch.int32)
     b200_out = model._wrap(words, counts, K, sizes, torch.device("cpu"))  # product code: packed buffer -> Instances
     from detectron2.structures import Boxes, Instances
-    from tridet.structures.boxes3d import Boxes3D
-    for o, r in zip(b200_out, ref_out):
+    from dd3d_b200.structures import Boxes3D
+    names = ["Car", "Pedestrian", "Cyclist", "Van", "Truck"]
+    rows = []
+    for b, o in enumerate(b200_out):
         inst = o["instances"]
         assert type(inst) is Instances and type(inst.pred_boxes) is Boxes and type(inst.pred_boxes3d) is Boxes3D
-        assert inst.image_size == r["instances"].image_size
-        assert set(inst.get_fields()) == set(r["instances"].get_fields())
-    rows = []
-    for out in (ref_out, b200_out):
-        ev = KITTI3DEvaluator("kitti_probe", iou_thresholds=[0.5, 0.7])
-        ev.reset()
-        ev.process(inputs, out)  # inference_on_dataset's per-batch call (scripts/train.py:228)
-        rows.append((ev._predictions_as_json, ev._predictions_kitti_format))
-    (ja, ka), (jb, kb) = rows
-    assert len(ja) == len(jb) == sum(int(c) for c in counts)
-    for a, b in zip(ja, jb):
-        assert a["category"] == b["category"] and a["file_name"] == b["file_name"] and a["image_id"] == b["image_id"]
-        np.testing.assert_allclose(a["bbox3d"], b["bbox3d"], rtol=1e-5, atol=1e-5)
-        np.testing.assert_allclose(a["bbox"], b["bbox"], rtol=1e-6, atol=1e-4)
-        assert abs(a["score"] - b["score"]) < 1e-6 and abs(a["score_3d"] - b["score_3d"]) < 1e-6
-    for fa, fb in zip(ka, kb):
-        assert fa.shape == fb.shape
-        assert list(fa[0]) == list(fb[0])  # class names
-        np.testing.assert_allclose(fa.iloc[:, 3:].to_numpy(dtype=np.float64), fb.iloc[:, 3:].to_numpy(dtype=np.float64),
-                                   rtol=1e-5, atol=1e-5)
-    print(f"BOUNDARY_OK detections={len(ja)} kitti_rows={sum(len(f) for f in ka)}")
+        assert tuple(inst.image_size) == tuple(ref[f"image_size{b}"].tolist())
+        assert sorted(inst.get_fields()) == ref[f"fields{b}"].tolist()
+        for i in range(len(inst)):  # the evaluator's per-detection reads (kitti_3d_evaluator.py:84-104)
+            x0, y0, x1, y1 = inst.pred_boxes.tensor[i].tolist()
+            rows.append(dict(category_id=int(inst.pred_classes[i]), category=names[int(inst.pred_classes[i])],
+                             bbox3d=inst.pred_boxes3d[i].vectorize()[0].numpy(), bbox=[x0, y0, x1 - x0, y1 - y0],
+                             score=float(inst.scores[i]), score_3d=float(inst.scores_3d[i]),
+                             file_name=f"img{b:06d}.png", image_id=b))
+    assert len(rows) == len(ref["category_id"]) == int(counts.sum())
+    for j, r in enumerate(rows):
+        assert r["category_id"] == ref["category_id"][j] and r["category"] == ref["category"][j]
+        assert r["file_name"] == ref["file_name"][j] and r["image_id"] == ref["image_id"][j]
+        np.testing.assert_allclose(r["bbox3d"], ref["bbox3d"][j], rtol=1e-5, atol=1e-5)
+        np.testing.assert_allclose(r["bbox"], ref["bbox"][j], rtol=1e-6, atol=1e-4)
+        assert abs(r["score"] - ref["score"][j]) < 1e-6 and abs(r["score_3d"] - ref["score_3d"][j]) < 1e-6
+    print(f"BOUNDARY_OK detections={len(rows)}")
 
 
 if __name__ == "__main__":

@@ -6,7 +6,6 @@ import pytest
 ROOT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..")
 sys.path.insert(0, os.path.abspath(ROOT))
 
-REFERENCE_ROOT = "/root/reference"
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
@@ -26,8 +25,3 @@ def pytest_collection_modifyitems(config, items):
     for item in items:
         if "gpu" in item.keywords:
             item.add_marker(skip)
-
-
-@pytest.fixture(scope="session")
-def have_reference():
-    return os.path.isdir(os.path.join(REFERENCE_ROOT, "tridet"))

@@ -1,15 +1,15 @@
 """dd3d_b200/config.py restates the reference's hydra config tree; this pins it: every key get_cfg() carries must equal the
 value hydra would resolve for the four shipped DD3D experiments (configs/experiments/dd3d_{kitti,nusc}_{dla34,v99}.yaml on
-top of configs/defaults.yaml), composed here with PyYAML + tests/hydra_lite.py (hydra-core is not installable offline).
-Needs /root/reference (build container only); the key list is also checked so config.py cannot silently drop a key the
-reference's DD3D.__init__ reads."""
+top of configs/defaults.yaml).  The resolved experiments are recorded in tests/golden/reference_configs.json, composed
+from the reference's config tree with PyYAML + tests/hydra_lite.py by oracle/gen_golden.py.  The key list is also checked
+so config.py cannot silently drop a key the reference's DD3D.__init__ reads."""
+import json
 import os
 
 import pytest
 
-from conftest import REFERENCE_ROOT
+from conftest import GOLDEN_DIR
 from dd3d_b200.config import get_cfg
-from hydra_lite import compose_experiment
 
 EXPERIMENTS = [  # experiment file, get_cfg arguments
     ("dd3d_kitti_dla34", dict(backbone="dla34", dataset="kitti_3d", meta_arch="DD3D")),
@@ -36,6 +36,11 @@ def _lookup(cfg, path):
     return cfg
 
 
+def reference_experiment(name):
+    with open(os.path.join(GOLDEN_DIR, "reference_configs.json")) as f:
+        return json.load(f)[name]
+
+
 def _same(a, b):
     if isinstance(a, (list, tuple)) and isinstance(b, (list, tuple)):
         return len(a) == len(b) and all(_same(x, y) for x, y in zip(a, b))
@@ -45,10 +50,8 @@ def _same(a, b):
 
 
 @pytest.mark.parametrize("experiment,args", EXPERIMENTS, ids=[e for e, _ in EXPERIMENTS])
-def test_config_equals_resolved_reference_experiment(experiment, args, have_reference):
-    if not have_reference:
-        pytest.skip("/root/reference not present")
-    ref = compose_experiment(os.path.join(REFERENCE_ROOT, "configs"), experiment)
+def test_config_equals_resolved_reference_experiment(experiment, args):
+    ref = reference_experiment(experiment)
     ours = get_cfg(**args)
     bad = []
     for path, val in _leaves(ours):
@@ -64,11 +67,9 @@ def test_config_equals_resolved_reference_experiment(experiment, args, have_refe
     assert not bad, "\n".join(f"{'.'.join(p)}: config.py {a!r} != reference {b!r}" for p, a, b in bad)
 
 
-def test_every_dd3d_key_of_the_reference_is_mirrored(have_reference):
+def test_every_dd3d_key_of_the_reference_is_mirrored():
     """DD3D.__init__ / the heads read cfg.DD3D.*, cfg.FE.*, cfg.MODEL.*: config.py must carry every leaf of those subtrees."""
-    if not have_reference:
-        pytest.skip("/root/reference not present")
-    ref = compose_experiment(os.path.join(REFERENCE_ROOT, "configs"), "dd3d_nusc_v99")
+    ref = reference_experiment("dd3d_nusc_v99")
     ours = get_cfg("v2_99", "nuscenes", meta_arch="NuscenesDD3D")
     missing = []
     for top in ("DD3D", "FE", "MODEL"):

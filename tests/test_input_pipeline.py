@@ -68,15 +68,12 @@ def test_shape_rule_and_cabi_agree():
         assert (nh.value, nw.value) == IO.resize_shortest_edge_shape(h, w, size, mx), (h, w, size, mx)
 
 
-def test_intrinsics_rescale_vs_live_reference(have_reference):
-    if not have_reference:
-        pytest.skip("/root/reference not present: covered by tests/golden/input_pipeline.npz")
-    from oracle import ref_standin
-    ref_standin.install()
-    from tridet.data.augmentations.resize_transform import ResizeTransform
+def test_intrinsics_rescale_vs_live_reference():
+    """The reference's ResizeTransform.apply_intrinsics on the two full-size shapes (reference_checks.npz)."""
+    g = np.load(os.path.join(GOLDEN_DIR, "reference_checks.npz"))
     K = np.float32([[1266.4, 0, 816.3], [0, 1266.4, 491.5], [0, 0, 1]])
-    for (h, w), (nh, nw) in [((900, 1600), (896, 1593)), ((375, 1242), (384, 1272))]:
-        assert np.array_equal(ResizeTransform(h, w, nh, nw).apply_intrinsics(K), IO.scale_intrinsics(K, h, w, nh, nw))
+    for i, ((h, w), (nh, nw)) in enumerate([((900, 1600), (896, 1593)), ((375, 1242), (384, 1272))]):
+        assert np.array_equal(g[f"intrinsics{i}/K"], IO.scale_intrinsics(K, h, w, nh, nw))
 
 
 # ------------------------------------------------------------------------------------------------ GPU
